@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/sec of the CLIP ViT-B/32 hot path (BASELINE.json configs[1]) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (uint8 frames -> transform -> ViT-B/32 tower -> (n,512) fp32 features)
 over one batch of 1000 synthetic 224x224x3 uint8 frames per GPU.  Prints ONE JSON line (rank 0):
@@ -12,6 +12,9 @@ over one batch of 1000 synthetic 224x224x3 uint8 frames per GPU.  Prints ONE JSO
   cpu_baseline  the oracle port (PIL transform + fp32 torch tower) timed on this box's host cores (N=1, rank 0)
 `--impl reference` times only that CPU path (the reference's `--cpu` path restated; see DESIGN.md) and prints the
 same line with "impl": "reference".
+`--dump-outputs DIR` writes what the timed path returned in its last timed step as DIR/<name>.npy (float32): the
+(n, 512) features (all ranks' rows, gathered, when N > 1; with --impl reference the first 32 frames' rows).  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -40,6 +43,7 @@ def emit(line: dict) -> None:
 
 
 FRAMES_PER_STEP = 1000
+REFERENCE_FRAMES_PER_STEP = 32           # --impl reference: frames of the 1000 the CPU oracle port runs per step
 METRIC = "frames/sec CLIP-ViT-B/32 @224px"
 UNIT = "frames/s"
 WORKLOAD = "CLIP-ViT-B/32 fix_2 on 1k synthetic 224x224 RGB frames (BASELINE.json configs[1])"
@@ -154,6 +158,15 @@ def synth_frames_host(n: int, seed: int):
     return torch.randint(0, 256, (n, 224, 224, 3), dtype=torch.uint8, generator=g)
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: one float32 DIR/<name>.npy per array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float32))
+
+
 def cpu_step(sd, frames_np):
     """The reference's per-video flow (models/CLIP/extract_clip.py:107-131) on the oracle port:
     PIL transform per frame -> stack -> fp32 tower -> numpy."""
@@ -189,31 +202,33 @@ def usable_cores() -> int:
     return max(1, n)
 
 
-def time_cpu(reps: int, warm: int, budget_s: float = 20.0):
-    """Times the oracle port on a bounded sample: the sample size is chosen from a probe so that warm-up + reps stay
-    near `budget_s` seconds of CPU work.  -> (per-rep seconds, cores, sample)"""
+def time_cpu(reps: int, warm: int, budget_s: float = 20.0, sample: int = 0):
+    """Times the oracle port on the first `sample` frames of the engine arm's rank-0 step (the same seeded frames, so
+    its features are rows 0 .. sample-1 of that step's).  sample = 0: chosen from a probe so that warm-up + reps stay
+    near `budget_s` seconds of CPU work.  -> (per-rep seconds, cores, sample, features of the last rep)"""
     import torch
     from video_features_b200 import synthetic_weights
     cores = usable_cores()
     torch.set_num_threads(cores)
     sd = synthetic_weights.clip_vit_b32_state_dict(0)
-    frames = synth_frames_host(256, 1234).numpy()
+    frames = synth_frames_host(FRAMES_PER_STEP, 100).numpy()
     cpu_step(sd, frames[:4])                                   # page in / thread pool start
-    t0 = time.perf_counter()
-    cpu_step(sd, frames[:16])
-    probe = max(time.perf_counter() - t0, 1e-3)
-    per_frame = probe / 16
-    sample = int(max(16, min(256, budget_s / max(reps + warm, 1) / per_frame)))
-    sample -= sample % 8
+    if not sample:
+        t0 = time.perf_counter()
+        cpu_step(sd, frames[:16])
+        probe = max(time.perf_counter() - t0, 1e-3)
+        per_frame = probe / 16
+        sample = int(max(16, min(256, budget_s / max(reps + warm, 1) / per_frame)))
+        sample -= sample % 8
     frames = frames[:sample]
     for _ in range(warm):
         cpu_step(sd, frames)
-    ts = []
+    ts, y = [], None
     for _ in range(reps):
         t0 = time.perf_counter()
-        cpu_step(sd, frames)
+        y = cpu_step(sd, frames)
         ts.append(time.perf_counter() - t0)
-    return ts, cores, sample
+    return ts, cores, sample, y
 
 
 def cpu_model_name() -> str:
@@ -229,8 +244,11 @@ def cpu_model_name() -> str:
 def run_reference(args, rank: int) -> None:
     if rank != 0:
         return
-    steps = min(max(args.steps, 1), 10)        # each step is a bounded sample; the whole arm stays within minutes
-    ts, cores, sample = time_cpu(steps, min(max(args.warmup, 1), 3), budget_s=30.0)
+    # each step is a fixed sample of the headline step's frames, so the arm's time grows linearly with --steps and its
+    # --dump-outputs rows are the same from run to run (and equal rows 0 .. sample-1 of the engine arm's dump)
+    ts, cores, sample, y = time_cpu(args.steps, min(max(args.warmup, 1), 3), sample=REFERENCE_FRAMES_PER_STEP)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"features": y})
     total = sum(ts)
     value = sample * len(ts) / total
     desc = (f"{sample} of the 1000 frames per step; PIL transform + fp32 torch tower (oracle port of the "
@@ -277,6 +295,7 @@ def run_engine(args, rank: int, world: int, local_rank: int) -> None:
     gathered = [torch.empty((world * n, 512), dtype=torch.float32, device=dev) for _ in range(2)] if world > 1 else None
     side = torch.cuda.Stream(device=dev) if world > 1 else None
     tick = [0]
+    last = {}
 
     def barrier():
         if world > 1:
@@ -296,6 +315,7 @@ def run_engine(args, rank: int, world: int, local_rank: int) -> None:
         y = eng.encode_frames_u8(frames_dev)
         if world > 1:
             gather_async(y)
+        last["y"] = y
         return y
 
     def step_host():
@@ -335,13 +355,15 @@ def run_engine(args, rank: int, world: int, local_rank: int) -> None:
         barrier()
         return float(ms.item())
 
-    W, K = max(args.warmup, 3), max(args.steps, 1)
+    W, K = max(args.warmup, 3), args.steps
     for _ in range(W):
         step_dev()
     launches0 = eng.launch_count
     sampler = ClockSampler(local_rank) if rank == 0 else None
     ms_total = timed(step_dev, K)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"features": gathered[(tick[0] - 1) & 1] if world > 1 else last["y"]})
     launches = (eng.launch_count - launches0) // K
     value = world * n * K / (ms_total / 1e3)
 
@@ -440,7 +462,7 @@ def run_engine(args, rank: int, world: int, local_rank: int) -> None:
         "roofline": roofline,
     }
     if rank == 0 and world == 1 and not args.no_cpu:
-        ts, cores, sample = time_cpu(3, 1, budget_s=20.0)
+        ts, cores, sample, _ = time_cpu(3, 1, budget_s=20.0)
         v = sample * len(ts) / sum(ts)
         line["cpu_baseline"] = {
             "value": v, "unit": UNIT, "cores": cores, "kind": "port",
@@ -516,15 +538,11 @@ RAFT_GFLOP_272x480 = 309.82                          # per pair, 20 iterations, 
 
 
 def _weights(kind: str):
-    """Reference checkpoint copy if present (checkpoints/), else seeded synthetic weights."""
-    import torch
-    p = os.path.join(ROOT, "checkpoints", {"rgb": "i3d_rgb.pt", "flow": "i3d_flow.pt", "raft": "raft-sintel.pth"}[kind])
-    if os.path.exists(p):
-        return torch.load(p, map_location="cpu"), "reference checkpoint"
-    from oracle import i3d_net
-    if kind == "raft":
-        raise SystemExit("bench --workload raft needs checkpoints/raft-sintel.pth (scripts/fetch_checkpoints.py)")
-    return i3d_net.synthetic_state_dict(kind, 0), "synthetic seed 0"
+    """Seeded stand-in of the reference's vendored checkpoint (oracle/checkpoint_standins.py): the same weights on every
+    machine, so runs are comparable; the time does not depend on the values."""
+    from oracle import checkpoint_standins
+    name = {"rgb": "i3d_rgb.pt", "flow": "i3d_flow.pt", "raft": "raft-sintel.pth"}[kind]
+    return checkpoint_standins.state_dict(name), f"seeded stand-in of {name} (per-tensor statistics of the vendored file)"
 
 
 def _timed_loop(fn, steps, warm):
@@ -985,7 +1003,13 @@ def main() -> None:
                          "/ c5 = configs[2] / configs[3] / configs[4] alone")
     ap.add_argument("--no-secondary", action="store_true", dest="no_secondary",
                     help="headline only: skip the secondary workloads (c5 video list, I3D, RAFT -> I3D flow)")
+    ap.add_argument("--dump-outputs", metavar="DIR", dest="dump_outputs",
+                    help="write the timed path's outputs of its last timed step to DIR/<name>.npy (clip workload)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload != "clip":
+        ap.error("--dump-outputs writes the headline path's outputs: use it with --workload clip")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -4,8 +4,9 @@ Follows models/raft/raft_src/: raft.py (InputPadder :27-44, RAFT.forward :115-17
 extractor.py (BasicEncoder :118-192, ResidualBlock :6-56), corr.py (CorrBlock :12-60, incl. the transposed 9x9
 window), update.py (BasicMotionEncoder :83-101, SepConvGRU :37-64, FlowHead :10-18, BasicUpdateBlock :118-139),
 utils/utils.py (bilinear_sampler :57-71, coords_grid :74-77).  Functional, driven by the checkpoint's own state dict
-(raft-sintel.pth, keys prefixed ``module.``).  Pinned against the reference module + vendored checkpoint run in the
-build container (scripts/make_golden.py -> tests/golden/raft_outputs.npz).
+(raft-sintel.pth, keys prefixed ``module.``).  Pinned against the reference module: bit-identical with the vendored
+checkpoint (scripts/make_golden.py raft -> tests/golden/raft_outputs.npz, kept as the record of that check) and on the
+checkpoint stand-in the tests use (scripts/make_golden.py standin -> tests/golden/standin_outputs.npz).
 """
 from __future__ import annotations
 

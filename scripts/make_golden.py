@@ -116,7 +116,10 @@ def main():
                                            (100, 60, 373, 224, Image.BICUBIC), (120, 160, 128, 170, Image.BILINEAR),
                                            (135, 240, 128, 227, Image.BILINEAR), (64, 48, 31, 17, Image.BICUBIC)]):
         im = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-        d[f"in{n}"] = im
+        if n == 4:      # replayed from the seed by the test instead of stored: keeps the file under 1 MB
+            d[f"shape{n}"] = np.array(im.shape, np.int64)
+        else:
+            d[f"in{n}"] = im
         d[f"out{n}"] = np.asarray(Image.fromarray(im).resize((ow, oh), f))
         d[f"filter{n}"] = np.int64(f)
     import PIL
@@ -226,3 +229,76 @@ def raft_golden():
 
 if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "raft":
     raft_golden()
+
+
+def checkpoint_stats():
+    """Per-tensor statistics of the reference's vendored checkpoints -> tests/golden/checkpoint_stats.npz, from which
+    oracle/checkpoint_standins.py draws seeded stand-ins (the checkpoints themselves are not part of the repository)."""
+    import torch
+    d = {}
+    for name, rel in (("i3d_rgb.pt", "models/i3d/checkpoints/i3d_rgb.pt"), ("i3d_flow.pt", "models/i3d/checkpoints/i3d_flow.pt"),
+                      ("raft-sintel.pth", "models/raft/checkpoints/raft-sintel.pth")):
+        sd = torch.load(os.path.join(REF, rel), map_location="cpu")
+        stats = []
+        for v in sd.values():
+            x = v.double()
+            stats.append([float(x.mean()), float(x.std()) if x.numel() > 1 else 0.0, float(x.min()), float(x.max()),
+                          float(v.is_floating_point())])
+        d[f"{name}/keys"] = np.array(list(sd))
+        d[f"{name}/ndim"] = np.array([v.dim() for v in sd.values()], np.int64)
+        d[f"{name}/dims"] = np.array([s for v in sd.values() for s in v.shape], np.int64)
+        d[f"{name}/stats"] = np.array(stats, np.float64)
+    np.savez_compressed(os.path.join(OUT, "checkpoint_stats.npz"), **d)
+
+
+def standin_golden():
+    """The reference's I3D and RAFT modules on the checkpoint stand-ins of oracle/checkpoint_standins.py, seeded inputs
+    (the same the tests draw) -> tests/golden/standin_outputs.npz.  The flow fields are kept on a strided grid (small
+    fixture); `raft_stride_<h>x<w>` records the stride."""
+    import torch
+    from oracle.checkpoint_standins import state_dict as checkpoint
+    sys.path.insert(0, REF)
+    cwd = os.getcwd()
+    os.chdir(REF)
+    try:
+        from models.i3d.i3d_src.i3d_net import I3D
+        from models.raft.raft_src.raft import RAFT, InputPadder
+        from oracle import i3d_net, raft_net
+        d = {}
+        for mod, cin in (("rgb", 3), ("flow", 2)):
+            sd = checkpoint(f"i3d_{mod}.pt")
+            net = I3D(num_classes=400, modality=mod).eval()
+            net.load_state_dict(sd)
+            for T in (16, 11):
+                x = torch.rand(1, cin, T, 224, 224, generator=torch.Generator().manual_seed(100 + T)) * 2 - 1
+                with torch.no_grad():
+                    y_ref = net(x, features=True)
+                rel = float((i3d_net.forward_features(sd, x) - y_ref).norm() / y_ref.norm())
+                print(f"i3d {mod} stand-in T={T}: oracle vs reference rel {rel:.2e}; |y| {float(y_ref.norm()):.3e}")
+                assert rel < 1e-5
+                d[f"i3d_{mod}_T{T}"] = y_ref.numpy()
+        sd = checkpoint("raft-sintel.pth")
+        net = torch.nn.DataParallel(RAFT(), device_ids=None)
+        net.load_state_dict(sd)
+        net = net.module.eval()
+        for (h, w, n, step) in RAFT_GOLDEN_CASES:
+            fr = raft_net.synthetic_frames(n, h, w, seed=h)
+            padder = InputPadder(fr.shape)
+            x = padder.pad(fr)
+            with torch.no_grad():
+                y_ref = net(x[:-1], x[1:], iters=20)
+            rel = float((raft_net.forward(sd, x[:-1], x[1:], 20) - y_ref).norm() / y_ref.norm())
+            print(f"raft stand-in {h}x{w}: oracle vs reference rel {rel:.2e}; mean |flow| {float(y_ref.abs().mean()):.3f}")
+            assert rel < 1e-4
+            d[f"raft_flow_{h}x{w}"] = padder.unpad(y_ref).numpy().astype(np.float32)[:, :, ::step, ::step]
+            d[f"raft_stride_{h}x{w}"] = np.int64(step)
+        np.savez_compressed(os.path.join(OUT, "standin_outputs.npz"), **d)
+    finally:
+        os.chdir(cwd)
+
+
+RAFT_GOLDEN_CASES = ((128, 160, 3, 4), (270, 480, 2, 6))       # (h, w, frames, stride of the stored grid)
+
+if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "standin":
+    checkpoint_stats()
+    standin_golden()

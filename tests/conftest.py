@@ -18,15 +18,6 @@ def pytest_configure(config):
         pass
 
 
-def pytest_sessionstart(session):
-    """The real-checkpoint parity tests never skip: in the build container the reference's vendored weights are copied
-    into ./checkpoints/ on demand (the GPU box receives that folder with the snapshot)."""
-    need = [os.path.join(ROOT, "checkpoints", n) for n in ("i3d_rgb.pt", "i3d_flow.pt", "raft-sintel.pth")]
-    if not all(os.path.exists(n) for n in need) and os.path.isdir("/root/reference/models"):
-        import subprocess
-        subprocess.call([sys.executable, os.path.join(ROOT, "scripts", "fetch_checkpoints.py")])
-
-
 @pytest.fixture(scope="session")
 def cuda_device():
     import torch

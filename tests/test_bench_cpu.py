@@ -8,9 +8,10 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _run(env_extra=None):
+def _run(env_extra=None, extra_args=()):
     env = dict(os.environ, **(env_extra or {}))
-    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1"],
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
+                        *extra_args],
                        capture_output=True, text=True, timeout=600, env=env, cwd=ROOT)
     assert p.returncode == 0, p.stderr[-2000:]
     return [l for l in p.stdout.splitlines() if l.strip()]
@@ -30,6 +31,29 @@ def test_reference_arm_prints_one_contract_line():
 def test_reference_arm_other_ranks_exit_without_work():
     lines = _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"})
     assert lines == []
+
+
+def test_reference_arm_dumps_the_last_step(tmp_path):
+    """--dump-outputs DIR: the features the timed path computed, float32, one row per frame of its fixed sample -- the
+    first 32 of the headline step's seeded frames (rank 0) -- equal to the oracle port run on those frames."""
+    import numpy as np
+    import torch
+    from oracle import clip_preprocess, clip_tower
+    from video_features_b200 import synthetic_weights
+    _run(extra_args=("--dump-outputs", str(tmp_path)))
+    y = np.load(tmp_path / "features.npy")
+    assert y.dtype == np.float32 and y.shape == (32, 512)
+    frames = torch.randint(0, 256, (1000, 224, 224, 3), dtype=torch.uint8, generator=torch.Generator().manual_seed(100))
+    with torch.no_grad():
+        ref = clip_tower.encode_image(synthetic_weights.clip_vit_b32_state_dict(0),
+                                      clip_preprocess.preprocess_batch(frames[:32].numpy())).numpy()
+    assert np.linalg.norm(y - ref) <= 1e-5 * np.linalg.norm(ref)
+
+
+def test_steps_below_one_are_rejected():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=600, cwd=ROOT)
+    assert p.returncode != 0 and "--steps" in p.stderr
 
 
 def test_engine_arm_fails_loudly_without_a_gpu():

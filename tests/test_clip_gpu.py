@@ -268,3 +268,23 @@ def test_b16_feature_type_through_extractor(cuda_device, tmp_path, monkeypatch):
     sd = synthetic_weights.clip_vit_b32_state_dict(9, patch=16)
     ref = clip_tower.encode_image(sd, clip_preprocess.preprocess_batch(frames))
     _check_rows(torch.from_numpy(np.asarray(feats)), ref)
+
+
+def test_bench_dump_outputs_are_the_headline_features(cuda_device, tmp_path):
+    """bench.py --dump-outputs: the (1000, 512) features of the last timed step, on the seeded frames of rank 0."""
+    import os
+    import subprocess
+    import sys
+    from oracle import clip_tower
+    from video_features_b200 import synthetic_weights
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    p = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "3", "--no-cpu",
+                        "--no-secondary", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert p.returncode == 0, p.stderr[-2000:]
+    y = np.load(tmp_path / "features.npy")
+    assert y.dtype == np.float32 and y.shape == (1000, 512)
+    frames = torch.randint(0, 256, (1000, 224, 224, 3), dtype=torch.uint8, generator=torch.Generator().manual_seed(100))
+    sd = synthetic_weights.clip_vit_b32_state_dict(0)
+    rows = [0, 1, 499, 998, 999]
+    ref = clip_tower.encode_image(sd, _transform_224(frames[rows]))
+    _check_rows(torch.from_numpy(y[rows]), ref)

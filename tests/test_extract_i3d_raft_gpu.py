@@ -1,5 +1,5 @@
-"""ExtractI3D / ExtractRAFT (reference-facing classes) on a synthetic video, real checkpoints, against the oracle run
-on the same decoded frames."""
+"""ExtractI3D / ExtractRAFT (reference-facing classes) on a synthetic video, seeded stand-ins of the reference's
+checkpoints (oracle/checkpoint_standins.py), against the oracle run on the same decoded frames."""
 import argparse
 import os
 
@@ -11,7 +11,14 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 import sys
 sys.path.insert(0, os.path.join(ROOT, "scripts", "precision"))
-from helpers import checkpoint  # noqa: E402  (a missing checkpoint copy FAILS these tests, it never skips them)
+from helpers import checkpoint  # noqa: E402
+
+
+@pytest.fixture
+def standin_checkpoints(monkeypatch):
+    """The extractors load the checkpoint stand-ins instead of files from $VF_CKPT_DIR / checkpoints/."""
+    from video_features_b200.extract import extract_i3d
+    monkeypatch.setattr(extract_i3d, "_STATE_DICTS", {k: checkpoint(n) for k, n in extract_i3d._CKPT.items()})
 
 
 def _write_video(path, n, h=120, w=160, fps=25.0, shift=(0.8, 0.5)):
@@ -35,15 +42,13 @@ def _ns(**kw):
 
 
 @pytest.mark.parametrize("clip,shift", [("low_motion", (0.8, 0.5)), ("high_motion", (4.5, -3.0))])
-def test_extract_i3d_two_streams_vs_oracle(cuda_device, tmp_path, clip, shift):
+def test_extract_i3d_two_streams_vs_oracle(cuda_device, standin_checkpoints, tmp_path, clip, shift):
     from PIL import Image
     from flow_quantiser_sensitivity import feature_sensitivity            # scripts/precision/
     from oracle import i3d_net, raft_net
     from video_features_b200 import utils
     from video_features_b200.extract.extract_i3d import ExtractI3D
     from video_features_b200.raft_engine import RAFTEngine
-    for n in ("i3d_rgb.pt", "i3d_flow.pt", "raft-sintel.pth"):
-        checkpoint(n)
     vid = str(tmp_path / "clip.mp4")
     _write_video(vid, 20, shift=shift)
     out = str(tmp_path / "out")
@@ -61,16 +66,16 @@ def test_extract_i3d_two_streams_vs_oracle(cuda_device, tmp_path, clip, shift):
     frames = [rd.get_frame(int(i)) for i in ix]
     rs = torch.stack([torch.from_numpy(np.asarray(Image.fromarray(f).resize((341, 256), Image.BILINEAR)).copy())
                       for f in frames]).permute(0, 3, 1, 2).float().to(cuda_device)
-    sd_rgb = {k: v.to(cuda_device) for k, v in torch.load(checkpoint("i3d_rgb.pt")).items()}
+    sd_rgb = {k: v.to(cuda_device) for k, v in checkpoint("i3d_rgb.pt").items()}
     ref_rgb = i3d_net.forward_features(sd_rgb, i3d_net.rgb_transform(rs[:-1]))
     rel = float((torch.from_numpy(res['rgb']).to(cuda_device) - ref_rgb).norm() / ref_rgb.norm())
     print(f"[{clip}] ExtractI3D rgb vs oracle:", rel)
     assert rel < 1e-3
-    sd_raft_cpu = torch.load(checkpoint("raft-sintel.pth"))
+    sd_raft_cpu = checkpoint("raft-sintel.pth")
     sd_raft = {k: v.to(cuda_device) for k, v in sd_raft_cpu.items()}
     xp = raft_net.pad(rs)
     flow = raft_net.forward(sd_raft, xp[:-1], xp[1:], 20)                # padded, never unpadded (extract_i3d.py:172)
-    sd_flow = {k: v.to(cuda_device) for k, v in torch.load(checkpoint("i3d_flow.pt")).items()}
+    sd_flow = {k: v.to(cuda_device) for k, v in checkpoint("i3d_flow.pt").items()}
     ref_flow = i3d_net.forward_features(sd_flow, i3d_net.flow_transform(flow))
     rel = float((torch.from_numpy(res['flow']).to(cuda_device) - ref_flow).norm() / ref_flow.norm())
     # The flow stream passes through the reference's 8-bit quantiser `round(128 + 255/40 f)` (transforms.py:43-51), a
@@ -98,15 +103,13 @@ def test_extract_i3d_two_streams_vs_oracle(cuda_device, tmp_path, clip, shift):
     assert rel <= bar, (rel, bar)
 
 
-def test_extract_i3d_mixed_aspect_ratios_and_precomputed_flow(cuda_device, tmp_path):
+def test_extract_i3d_mixed_aspect_ratios_and_precomputed_flow(cuda_device, standin_checkpoints, tmp_path):
     """(a) a list whose second video is wider than the first: the RAFT engine's workspace must follow (the reference
     handles any resolution per video); (b) --flow_type flow: pre-computed flow_x / flow_y jpg pairs
     (extract_i3d.py:195-229,266-278) against the oracle fed with the very same jpgs."""
     import cv2
     from oracle import i3d_net
     from video_features_b200.extract.extract_i3d import ExtractI3D
-    for n in ("i3d_rgb.pt", "i3d_flow.pt", "raft-sintel.pth"):
-        checkpoint(n)
     a, b = str(tmp_path / "narrow.mp4"), str(tmp_path / "wide.mp4")
     _write_video(a, 14, h=120, w=160)                     # -> 256x341
     _write_video(b, 14, h=96, w=192)                      # -> 256x512: wider than the engine created for `a`
@@ -132,7 +135,7 @@ def test_extract_i3d_mixed_aspect_ratios_and_precomputed_flow(cuda_device, tmp_p
     assert got['flow'].shape == (1, 1024) and got['rgb'].shape == (1, 1024)
     imgs = torch.stack([torch.stack([torch.from_numpy(cv2.imread(str(fdir / f"flow_{c}_{i:05d}.jpg"), cv2.IMREAD_GRAYSCALE))
                                      for c in "xy"]) for i in range(12)])            # uint8 (12,2,256,344), as mmcv.imread
-    sd_flow = {k: v.to(cuda_device) for k, v in torch.load(checkpoint("i3d_flow.pt")).items()}
+    sd_flow = {k: v.to(cuda_device) for k, v in checkpoint("i3d_flow.pt").items()}
     # the reference applies its flow transform to these uint8 grey levels as they are: clamp(-20,20) keeps [0,20]
     ref = i3d_net.forward_features(sd_flow, i3d_net.flow_transform(imgs.float().to(cuda_device)))
     rel = float((torch.from_numpy(got['flow']).to(cuda_device) - ref).norm() / ref.norm())
@@ -140,9 +143,8 @@ def test_extract_i3d_mixed_aspect_ratios_and_precomputed_flow(cuda_device, tmp_p
     assert rel < 1e-3
 
 
-def test_extract_raft_writes_flow(cuda_device, tmp_path):
+def test_extract_raft_writes_flow(cuda_device, standin_checkpoints, tmp_path):
     from oracle import raft_net
-    checkpoint("raft-sintel.pth")
     from video_features_b200.extract.extract_raft import ExtractRAFT
     vid = str(tmp_path / "clip2.mp4")
     _write_video(vid, 6, h=128, w=160)
@@ -160,7 +162,7 @@ def test_extract_raft_writes_flow(cuda_device, tmp_path):
             break
         fr.append(cv2.cvtColor(f, cv2.COLOR_BGR2RGB))
     x = torch.from_numpy(np.stack(fr)).permute(0, 3, 1, 2).float().to(cuda_device)
-    sd = {k: v.to(cuda_device) for k, v in torch.load(checkpoint("raft-sintel.pth")).items()}
+    sd = {k: v.to(cuda_device) for k, v in checkpoint("raft-sintel.pth").items()}
     ref = raft_net.forward(sd, x[:-1], x[1:], 20).cpu().numpy()
     rel = np.linalg.norm(flow - ref) / np.linalg.norm(ref)
     print("ExtractRAFT vs oracle:", rel)

@@ -1,13 +1,14 @@
 """RAFT flow through the C ABI against the fp32 oracle (oracle/raft_net.py, pinned bit-for-bit to the reference
-module) and against the reference module's own output (tests/golden/raft_outputs.npz).
+module) and against the reference module's own output (tests/golden/standin_outputs.npz).
 
 Bar (SURVEY 8d): rel-L2 <= 1e-3 and max-abs <= 1e-3 * max|ref| on the flow field.  RAFT's 20 refinement steps amplify
 operand rounding by two to three orders of magnitude on hard inputs (the fp32 oracle itself moves by 2.5e-5 between 1
 and 16 CPU threads on block-compressed frames), so the engine carries EVERY GEMM operand as a split-fp16 pair
 (activations [hi | lo] with duplicated weight columns, weights as hi + lo passes, DESIGN.md §2).  Measured: rel-L2
 5.5e-6 / max 3.8e-5 at 128x160, 1.7e-5 / 1.8e-4 at 270x480, 5.7e-5 on block-compressed video
-(test_extract_i3d_raft_gpu.py) -- both parts of the bar are met with margin.  Needs the reference checkpoint copy
-under checkpoints/ (scripts/fetch_checkpoints.py) -- RAFT with random weights is not a meaningful dynamical system."""
+(test_extract_i3d_raft_gpu.py) -- both parts of the bar are met with margin.  (Those figures are for the vendored
+raft-sintel.pth.)  The weights are a seeded stand-in of that checkpoint (oracle/checkpoint_standins.py): plain random
+weights make RAFT's iteration chaotic, so the stand-in damps the flow head to keep it well conditioned."""
 import os
 
 import numpy as np
@@ -18,7 +19,6 @@ import video_features_b200  # noqa: F401
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CKPT = os.path.join(ROOT, "checkpoints", "raft-sintel.pth")
 
 
 def _err(y, ref):
@@ -29,9 +29,8 @@ def _err(y, ref):
 @pytest.fixture(scope="module")
 def raft(cuda_device):
     from helpers import checkpoint
-    checkpoint("raft-sintel.pth")                      # fails (never skips) when the copy is missing
     from video_features_b200.raft_engine import RAFTEngine
-    sd = torch.load(CKPT, map_location="cpu")
+    sd = checkpoint("raft-sintel.pth")
     eng = RAFTEngine(sd, 0, max_frames=5, max_h=272, max_w=480)
     yield sd, eng
     eng.close()
@@ -52,7 +51,8 @@ def test_raft_stages_and_one_iteration(raft, cuda_device):
     cnet = R.encoder(sdg, "cnet", img[:-1], "batch")
     e2 = _err(eng.debug_read(1), cnet)
     print("cnet output:", e2)
-    assert e[0] < 1e-4 and e2[0] < 1e-4         # measured 3.8e-6 / 6.8e-6
+    # measured on a B200 with the stand-in: 5.6e-6 / 2.0e-6 (vendored checkpoint: 3.8e-6 / 6.8e-6)
+    assert e[0] < 1e-4 and e2[0] < 1e-4
     # first lookup (coords = grid) against the oracle's pyramid lookup
     pyr = R.corr_pyramid(fmap[:-1].float(), fmap[1:].float())
     H8, W8 = 16, 20
@@ -62,14 +62,14 @@ def test_raft_stages_and_one_iteration(raft, cuda_device):
     eng.flow(x, iters=1, unpad=False)
     e = _err(eng.debug_read(4), look)       # (the last lookup of a 1-iteration run is the first one)
     print("corr lookup:", e)
-    assert e[0] < 1e-4
+    assert e[0] < 1e-4                          # measured with the stand-in: 3.5e-6
     ref1, low1 = R.forward(sd_to(sd, cuda_device), x[:-1], x[1:], 1, return_lowres=True)
     e = _err(eng.debug_read(3), low1)
     print("low-res flow after 1 iteration:", e)
-    assert e[0] < 1e-4
+    assert e[0] < 1e-4                          # measured with the stand-in: 1.9e-5
     e = _err(y1, ref1)
     print("flow_up after 1 iteration:", e)
-    assert e[0] < 1e-4 and e[1] < 1e-3
+    assert e[0] < 1e-4 and e[1] < 1e-3          # measured with the stand-in: 4.9e-5 / 1.8e-4
 
 
 def test_raft_odd_map_size(raft, cuda_device):
@@ -81,7 +81,7 @@ def test_raft_odd_map_size(raft, cuda_device):
     ref = R.forward(sd_to(sd, cuda_device), x[:-1], x[1:], 12)
     rel, mx = _err(y, ref)
     print(f"200x200: rel-L2 {rel:.3e} max {mx:.3e}")
-    assert torch.isfinite(y).all() and rel < 1e-4 and mx < 1e-3
+    assert torch.isfinite(y).all() and rel < 1e-4 and mx < 1e-3     # measured with the stand-in: 2.6e-5 / 1.4e-4
 
 
 def sd_to(sd, dev):
@@ -102,10 +102,13 @@ def test_raft_20_iterations_vs_oracle_and_reference_golden(raft, cuda_device, h,
     d = (y.double().cpu() - ref.double().cpu()).abs().flatten()
     print(f"    abs err px: max {float(d.max()):.4f}  p99.9 {float(d.kthvalue(int(d.numel() * 0.999)).values):.4f}  "
           f"median {float(d.median()):.5f}  (max |flow| {float(ref.abs().max()):.3f})")
-    assert rel < 1e-4            # north-star bar 1e-3; measured 5.5e-6 / 1.7e-5
-    assert mx < 1e-3             # the north-star max-abs bar; measured 3.8e-5 / 1.8e-4
-    gold = np.load(os.path.join(ROOT, "tests", "golden", "raft_outputs.npz"))[f"flow_{h}x{w}"]
-    got = y.cpu().numpy() if h < 200 else y.cpu().numpy()[:, :, ::3, ::3]
+    # north-star bars 1e-3; measured on a B200 with the stand-in: rel 3.0e-5 / 2.1e-5 (vendored checkpoint: 5.5e-6 /
+    # 1.7e-5), max-abs 1.6e-4 / 1.4e-4 (vendored: 3.8e-5 / 1.8e-4)
+    assert rel < 1e-4
+    assert mx < 1e-3
+    fixture = np.load(os.path.join(ROOT, "tests", "golden", "standin_outputs.npz"))
+    gold, stride = fixture[f"raft_flow_{h}x{w}"], int(fixture[f"raft_stride_{h}x{w}"])     # a strided grid of the flow
+    got = y.cpu().numpy()[:, :, ::stride, ::stride]
     rel_g = float(np.linalg.norm(got - gold) / np.linalg.norm(gold))
     print(f"{h}x{w}: vs reference-module golden rel-L2 {rel_g:.3e}")
     assert rel_g < 1e-4

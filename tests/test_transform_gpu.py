@@ -18,14 +18,11 @@ def _resize(img: np.ndarray, oh: int, ow: int, filt: int) -> np.ndarray:
 
 
 def test_resize_matches_pillow_fixture(cuda_device):
-    g = np.load(os.path.join(GOLD, "pillow_resize.npz"))
-    n = 0
-    while f"in{n}" in g:
-        out = g[f"out{n}"]
-        got = _resize(g[f"in{n}"], out.shape[0], out.shape[1], int(g[f"filter{n}"]))
-        assert np.array_equal(got, out), f"case {n}"
-        n += 1
-    assert n >= 5
+    from helpers import pillow_resize_cases
+    cases = pillow_resize_cases()
+    for n, (im, out, filt) in enumerate(cases):
+        assert np.array_equal(_resize(im, out.shape[0], out.shape[1], filt), out), f"case {n}"
+    assert len(cases) >= 6
 
 
 def test_resize_matches_reference_i3d_chain_fixture(cuda_device):
