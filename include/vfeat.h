@@ -216,6 +216,32 @@ int vf_raft_padded_size(int Hs, int Ws, int* H, int* W);
 int vf_raft_debug_read(vf_raft_t* h, int what, float* out, int64_t capacity, int* dims4, void* stream);
 int64_t vf_raft_launch_count(const vf_raft_t* h);
 
+/* ---- ResNet-18/34/50/101/152 frame features: replaces `model(batch)` with
+ * model = torchvision.models.resnet{depth}(pretrained=True), eval, fc = Identity (models/resnet/extract_resnet.py:54-71,
+ * called at :109).  Weights: torchvision's state_dict tensors by name ("conv1.weight", "layer1.0.bn1.running_var", ...),
+ * HOST fp32; num_batches_tracked and fc.* are not read. */
+typedef struct vf_resnet vf_resnet_t;
+/* Workspace for max_frames frames per chunk; a call with more frames runs in equal chunks. */
+int vf_resnet_create(vf_resnet_t** out, int depth, const vf_named_tensor* tensors, int n_tensors, int device, int max_frames);
+int vf_resnet_destroy(vf_resnet_t* h);
+/* 512 (depth 18, 34) or 2048 (50, 101, 152) */
+int vf_resnet_feature_dim(const vf_resnet_t* h);
+/* frames: n x 3 x 224 x 224 fp32 on the device, normalised (extract_resnet.py:106-109 `model(batch)`);
+ * out: n x feature_dim fp32 on the device. */
+int vf_resnet_forward_f32(vf_resnet_t* h, const float* frames, int n, float* out, void* stream);
+/* frames: n x src_h x src_w x 3 uint8 on the device -> Resize(256, Pillow bilinear) -> CenterCrop(224) -> ToTensor ->
+ * Normalize(ImageNet) -> net (extract_resnet.py:32-38 then :109); swap_rb: the frames are BGR (cv2) and are read as
+ * RGB (extract_resnet.py:142). */
+int vf_resnet_forward_u8(vf_resnet_t* h, const uint8_t* frames, int n, int src_h, int src_w, int swap_rb, float* out,
+                         void* stream);
+/* CenterCrop(224) -> ToTensor -> Normalize(ImageNet mean / std) of n resized uint8 HWC frames (extract_resnet.py:35-37)
+ * -> n x 3 x 224 x 224 fp32 on the device; swap_rb as above. */
+int vf_imagenet_normalize_u8(const uint8_t* src, int n, int src_h, int src_w, int swap_rb, float* dst, void* stream);
+/* Diagnostics: a stage output of the last chunk of the last call as fp32 NCHW; stage 0 = stem + max pool (64 x 56 x
+ * 56), 1..4 = layer1..4.  out = NULL only fills dims4. */
+int vf_resnet_read_stage(vf_resnet_t* h, int stage, float* out, int64_t capacity, int* dims4, void* stream);
+int64_t vf_resnet_launch_count(const vf_resnet_t* h);
+
 #ifdef __cplusplus
 }
 #endif

@@ -10,7 +10,8 @@ import torch  # noqa: F401
 
 from video_features_b200.utils import form_list_from_user_input, sanity_check
 
-SUPPORTED = ['i3d', 'raft', 'CLIP-ViT-B/32', 'CLIP-ViT-B/16', 'CLIP4CLIP-ViT-B-32']
+SUPPORTED = ['i3d', 'raft', 'CLIP-ViT-B/32', 'CLIP-ViT-B/16', 'CLIP4CLIP-ViT-B-32', 'resnet18', 'resnet34', 'resnet50',
+             'resnet101', 'resnet152']
 
 
 def build_extractor(args):
@@ -24,8 +25,10 @@ def build_extractor(args):
     if args.feature_type == 'raft':
         from video_features_b200.extract.extract_raft import ExtractRAFT
         return ExtractRAFT(args)
-    if args.feature_type in ['vggish', 'r21d_rgb', 'resnet18', 'resnet34', 'resnet50', 'resnet101', 'resnet152', 'pwc',
-                             'vggish_torch']:
+    if args.feature_type in ['resnet18', 'resnet34', 'resnet50', 'resnet101', 'resnet152']:
+        from video_features_b200.extract.extract_resnet import ExtractResNet
+        return ExtractResNet(args)
+    if args.feature_type in ['vggish', 'r21d_rgb', 'pwc', 'vggish_torch']:
         raise NotImplementedError(f'{args.feature_type}: outside the hot path this engine rebuilds (SURVEY.md §2)')
     raise NotADirectoryError                      # main.py:41
 
@@ -77,13 +80,13 @@ _FLAGS = [
     ('--on_extraction', dict(default='print', choices=['print', 'save_numpy', 'save_pickle'], help='sink of the features')),
     ('--output_path', dict(default='./output', help='root of the saved features')),
     ('--output_direct', dict(action='store_true', help='save as <output_path>/<video stem>.npy')),
-    ('--extraction_fps', dict(type=float, help='resample to this frame rate first (I3D)')),
+    ('--extraction_fps', dict(type=float, help='resample to this frame rate first (I3D; refused by RAFT and ResNet)')),
     ('--extract_method', dict(type=str, help='frame sampler: uni_N or fix_N')),
     ('--stack_size', dict(type=int, help='frames per I3D stack')),
     ('--step_size', dict(type=int, help='frames between I3D stacks')),
     ('--streams', dict(nargs='+', choices=['flow', 'rgb'], help='I3D streams (default: both)')),
     ('--flow_type', dict(choices=['raft', 'pwc', 'flow'], default='pwc', help='optical flow feeding the I3D flow stream')),
-    ('--batch_size', dict(type=int, default=1, help='frame pairs per RAFT call')),
+    ('--batch_size', dict(type=int, default=1, help='frame pairs per RAFT call, frames per ResNet call')),
     ('--resize_to_larger_edge', dict(dest='resize_to_smaller_edge', action='store_false', default=True,
                                     help='--side_size applies to the larger edge instead of the smaller one')),
     ('--side_size', dict(type=int, help='RAFT: resize frames to this edge length first')),

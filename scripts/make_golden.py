@@ -302,3 +302,50 @@ RAFT_GOLDEN_CASES = ((128, 160, 3, 4), (270, 480, 2, 6))       # (h, w, frames, 
 if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "standin":
     checkpoint_stats()
     standin_golden()
+
+
+RESNET_GEOMETRIES = ((240, 320), (320, 240), (180, 200))   # the sample video's size, a portrait frame, an up-scale
+RESNET_FRAME_SEED, RESNET_INPUT_SEED, RESNET_WEIGHT_SEED = 21, 5, 0
+
+
+def resnet_frames(h, w, seed=RESNET_FRAME_SEED):
+    """The uint8 RGB frame the transform fixture is computed on (regenerated by the tests)."""
+    return np.random.default_rng([seed, h, w]).integers(0, 256, (h, w, 3), dtype=np.uint8)
+
+
+def resnet_input():
+    import torch
+    return torch.randn(2, 3, 224, 224, generator=torch.Generator().manual_seed(RESNET_INPUT_SEED))
+
+
+def resnet_golden():
+    """torchvision itself (the reference runs torchvision.models.resnet{depth} and torchvision.transforms,
+    models/resnet/extract_resnet.py:32-38,54-71): the features of all five depths with fc = Identity on seeded weights
+    and seeded inputs, and the sha256 of the transform's fp32 output bytes on three frame geometries."""
+    import hashlib
+    import torch
+    import torchvision
+    import torchvision.transforms as T
+    from video_features_b200 import synthetic_weights as sw
+    d = {}
+    x = resnet_input()
+    for depth in (18, 34, 50, 101, 152):
+        m = getattr(torchvision.models, f"resnet{depth}")()
+        m.load_state_dict(sw.resnet_state_dict(depth, RESNET_WEIGHT_SEED))
+        m.fc = torch.nn.Identity()
+        m.eval()
+        with torch.no_grad():
+            d[f"resnet{depth}"] = m(x).numpy()
+    tf = T.Compose([T.ToPILImage(), T.Resize(256), T.CenterCrop(224), T.ToTensor(),
+                    T.Normalize(mean=[0.485, 0.456, 0.406], std=[0.229, 0.224, 0.225])])
+    for h, w in RESNET_GEOMETRIES:
+        y = tf(resnet_frames(h, w)).numpy()
+        assert y.dtype == np.float32 and y.shape == (3, 224, 224)
+        d[f"transform_{h}x{w}_sha256"] = np.array(hashlib.sha256(np.ascontiguousarray(y).tobytes()).hexdigest())
+        d[f"transform_{h}x{w}_sum"] = np.float64(y.astype(np.float64).sum())
+    d["torchvision_version"] = np.array(torchvision.__version__)
+    np.savez_compressed(os.path.join(OUT, "resnet_outputs.npz"), **d)
+
+
+if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "resnet":
+    resnet_golden()

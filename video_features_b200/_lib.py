@@ -103,6 +103,14 @@ SIGNATURES = {
     "vf_raft_padded_size": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "vf_raft_debug_read": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.POINTER(C.c_int), C.c_void_p]),
     "vf_raft_launch_count": (C.c_int64, [C.c_void_p]),
+    "vf_resnet_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(NamedTensor), C.c_int, C.c_int, C.c_int]),
+    "vf_resnet_destroy": (C.c_int, [C.c_void_p]),
+    "vf_resnet_feature_dim": (C.c_int, [C.c_void_p]),
+    "vf_resnet_forward_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "vf_resnet_forward_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "vf_imagenet_normalize_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "vf_resnet_read_stage": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.POINTER(C.c_int), C.c_void_p]),
+    "vf_resnet_launch_count": (C.c_int64, [C.c_void_p]),
     "vf_clip_profile": (C.c_int, [C.c_void_p, C.c_int]),
     "vf_clip_profile_categories": (C.c_int, [C.c_void_p, C.POINTER(C.c_double)]),
     "vf_clip_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int64),

@@ -8,6 +8,15 @@
 
 namespace vf {
 
+// torchvision ToTensor + Normalize(ImageNet mean / std) of one uint8 value of channel c: float32(v) / 255, then
+// (x - mean) / std -- IEEE fp32 ops in torchvision's order, constants float32-rounded as torch does.  The ResNet
+// extractor's transform (reference: models/resnet/extract_resnet.py:32-38).
+__device__ __forceinline__ float imagenet_norm(uint8_t v, int c) {
+    const float mean = c == 0 ? 0.485f : (c == 1 ? 0.456f : 0.406f);
+    const float std = c == 0 ? 0.229f : (c == 1 ? 0.224f : 0.225f);
+    return __fdiv_rn(__fsub_rn(__fdiv_rn(float(v), 255.0f), mean), std);
+}
+
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }

@@ -88,6 +88,9 @@ int launch_clip_patchify(const uint8_t* src, int n, int src_h, int src_w, int cr
 int launch_clip_patchify_f32(const float* src_chw, int n, __half* patches, int patch, cudaStream_t s);
 int launch_clip_normalize_f32(const uint8_t* src, int n, int src_h, int src_w, int crop_y, int crop_x, float* dst_chw,
                               cudaStream_t s);
+// the same with torchvision's ImageNet mean / std (ResNet); swap_rb reads BGR frames as RGB
+int launch_imagenet_normalize_f32(const uint8_t* src, int n, int src_h, int src_w, int crop_y, int crop_x, int swap_rb,
+                                  float* dst_chw, cudaStream_t s);
 // x (+= y) ; out = LayerNorm(x) -- rows of 768 fp32.  y may be null; write_x stores the summed residual stream back.
 int launch_add_layernorm(float* x, int64_t x_row_stride, const __half* y, int64_t y_row_stride, int write_x,
                          const float* gamma, const float* beta, void* out, int64_t out_row_stride, int out_f32, int rows,

@@ -77,9 +77,18 @@ __global__ void clip_patchify_f32_kernel(const float* __restrict__ src, int n, _
         make_uint4(pack_half2(a.x, a.y), pack_half2(a.z, a.w), pack_half2(d.x, d.y), pack_half2(d.z, d.w));
 }
 
-// uint8 HWC (crop window) -> fp32 CHW normalised: the tensor the reference feeds encode_image. 4 px / thread.
-__global__ void clip_normalize_f32_kernel(const uint8_t* __restrict__ src, int n, int src_h, int src_w, int cy, int cx,
-                                          float* __restrict__ dst) {
+struct ClipNorm {
+    __device__ static float apply(uint8_t v, int c) { return clip_norm(v, c); }
+};
+struct ImageNetNorm {
+    __device__ static float apply(uint8_t v, int c) { return imagenet_norm(v, c); }
+};
+
+// uint8 HWC (crop window) -> fp32 CHW normalised: the tensor the reference feeds the network. 4 px / thread.
+// swap_rb: read the source's channels in reverse order (BGR frames -> RGB values)
+template <class Norm>
+__global__ void normalize_f32_kernel(const uint8_t* __restrict__ src, int n, int src_h, int src_w, int cy, int cx,
+                                     int swap_rb, float* __restrict__ dst) {
     const int64_t idx = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
     const int64_t total = int64_t(n) * 224 * 56;
     if (idx >= total) return;
@@ -92,8 +101,9 @@ __global__ void clip_normalize_f32_kernel(const uint8_t* __restrict__ src, int n
     for (int i = 0; i < 12; ++i) px[i] = __ldg(p + i);
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        float4 v = make_float4(clip_norm(px[c], c), clip_norm(px[3 + c], c), clip_norm(px[6 + c], c),
-                               clip_norm(px[9 + c], c));
+        const int sc = swap_rb ? 2 - c : c;
+        float4 v = make_float4(Norm::apply(px[sc], c), Norm::apply(px[3 + sc], c), Norm::apply(px[6 + sc], c),
+                               Norm::apply(px[9 + sc], c));
         *reinterpret_cast<float4*>(dst + ((int64_t(b) * 3 + c) * 224 + y) * 224 + xg * 4) = v;
     }
 }
@@ -612,7 +622,15 @@ int launch_clip_patchify_f32(const float* src_chw, int n, __half* patches, int p
 int launch_clip_normalize_f32(const uint8_t* src, int n, int src_h, int src_w, int crop_y, int crop_x, float* dst_chw,
                               cudaStream_t s) {
     const int64_t total = int64_t(n) * 224 * 56;
-    clip_normalize_f32_kernel<<<blocks_for(total, 256), 256, 0, s>>>(src, n, src_h, src_w, crop_y, crop_x, dst_chw);
+    normalize_f32_kernel<ClipNorm><<<blocks_for(total, 256), 256, 0, s>>>(src, n, src_h, src_w, crop_y, crop_x, 0, dst_chw);
+    VF_CUDA(cudaGetLastError());
+    return VF_OK;
+}
+int launch_imagenet_normalize_f32(const uint8_t* src, int n, int src_h, int src_w, int crop_y, int crop_x, int swap_rb,
+                                  float* dst_chw, cudaStream_t s) {
+    const int64_t total = int64_t(n) * 224 * 56;
+    normalize_f32_kernel<ImageNetNorm><<<blocks_for(total, 256), 256, 0, s>>>(src, n, src_h, src_w, crop_y, crop_x, swap_rb,
+                                                                             dst_chw);
     VF_CUDA(cudaGetLastError());
     return VF_OK;
 }

@@ -28,19 +28,10 @@
 #include <vector>
 
 #include "internal.h"
+#include "conv2d.h"
 #include "raft_kernels.h"
 
 namespace vf {
-
-struct ConvW {       // a convolution prepared for conv_gemm_f16
-    int n_out = 0;          // GEMM N (padded to a multiple of 8)
-    int ntaps = 0, k_per_tap = 0;
-    std::vector<int> dh, dw0;   // per tap: row offset (in kernel rows) and the column shift of its first element
-    int nsplit = 1;             // 2: w = [hi (ntaps*k_per_tap) | lo (same)] along K (ConvGeom::nsplit)
-    unsigned long long lo_mask = 0;   // K blocks (per tap) holding only lo-half activation columns (ConvGeom::lo_mask)
-    __half* w = nullptr;
-    float *scale = nullptr, *bias = nullptr;
-};
 
 static const int HX = RAFT_HX;   // hx / qx row layout: raft_kernels.h
 static const int CF = RAFT_CF;    // correlation-feature rows: raft_kernels.h
@@ -52,8 +43,9 @@ using namespace vf;
 struct vf_raft {
     int device = 0, max_frames = 0, max_h = 0, max_w = 0;
     int lead_alloc = 0;         // guard rows in front of every update-block buffer (pointers below are past them)
-    int wsplit = 2;             // weights as hi+lo fp16 pairs (VF_RAFT_FAST=1: single fp16 weights, outside the parity bar)
     std::vector<void*> allocs;
+    ConvAlloc ca;               // weight uploads: ralloc into `allocs`; wsplit 2 = weights as hi+lo fp16 pairs
+                                // (VF_RAFT_FAST=1: single fp16 weights, outside the parity bar)
     // encoders: [0] = fnet (instance norm), [1] = cnet (batch norm folded)
     struct Enc {
         ConvW conv1, l1[4], l2c1, l2down, l2[3], l3c1, l3down, l3[3], conv2;
@@ -95,166 +87,6 @@ static int ralloc(vf_raft* h, Tp** p, size_t count) {
     return VF_OK;
 }
 
-struct TensorTable {
-    const vf_named_tensor* t; int n;
-    const float* get(const std::string& name, int64_t numel) const {
-        for (int i = 0; i < n; ++i)
-            if (name == t[i].name) return t[i].numel == numel ? t[i].data : nullptr;
-        return nullptr;
-    }
-};
-
-// Generic filter re-layout.  w: [co][ci][kh][kw]; col(dh, dw, c) -> K column or -1.  Output rows padded to n_out.
-// col_lo (optional): a second K column receiving the same weight -- the column of the operand's lo half when the
-// activation is stored as a split-fp16 pair.
-static int upload_conv(vf_raft* h, ConvW& cw, const float* w, const float* b, int co, int ci, int kh, int kw, int n_out,
-                       int Ktot, const std::function<int(int, int, int)>& col, const float* bn_scale,
-                       const float* bn_shift, float extra_scale,
-                       const std::function<int(int, int, int)>& col_lo = nullptr, int nsplit = -1) {
-    if (nsplit < 0) nsplit = h->wsplit;
-    cw.nsplit = nsplit;
-    const size_t Kall = size_t(Ktot) * nsplit;
-    std::vector<__half> B(size_t(n_out) * Kall, __float2half_rn(0.f));
-    std::vector<char> has_hi(size_t(Ktot), 0);      // K columns that multiply a hi (or single-fp16) activation
-    for (int o = 0; o < co; ++o)
-        for (int c = 0; c < ci; ++c)
-            for (int a = 0; a < kh; ++a)
-                for (int d = 0; d < kw; ++d) {
-                    const int k = col(a, d, c);
-                    if (k < 0) continue;
-                    if (k >= Ktot) return fail(VF_ERR_INVALID, "raft_create: filter column out of range");
-                    const float wf = w[((size_t(o) * ci + c) * kh + a) * kw + d];
-                    const __half wv = __float2half_rn(wf);
-                    const __half wl = __float2half_rn(wf - __half2float(wv));
-                    B[size_t(o) * Kall + k] = wv;
-                    has_hi[k] = 1;
-                    if (nsplit == 2) B[size_t(o) * Kall + Ktot + k] = wl;
-                    if (col_lo) {
-                        const int k2 = col_lo(a, d, c);
-                        if (k2 >= Ktot) return fail(VF_ERR_INVALID, "raft_create: filter column out of range");
-                        if (k2 >= 0) {
-                            B[size_t(o) * Kall + k2] = wv;
-                            if (nsplit == 2) B[size_t(o) * Kall + Ktot + k2] = wl;
-                        }
-                    }
-                }
-    std::vector<float> sc(n_out, 0.f), bi(n_out, 0.f);
-    for (int o = 0; o < co; ++o) {
-        const float s = (bn_scale ? bn_scale[o] : 1.f) * extra_scale;
-        sc[o] = s;
-        bi[o] = (b ? b[o] : 0.f) * s + (bn_shift ? bn_shift[o] : 0.f) * extra_scale;
-    }
-    cw.n_out = n_out;
-    // a K block none of whose columns meets a hi half needs only the W_hi pass (a_lo . w_lo < 2^-22 of the product)
-    cw.lo_mask = 0;
-    const int kpt_blocks = (cw.k_per_tap + 63) / 64;
-    if (nsplit == 2 && kpt_blocks <= 64 && cw.ntaps * cw.k_per_tap == Ktot) {
-        unsigned long long m = ~0ull;
-        for (int t = 0; t < cw.ntaps; ++t)
-            for (int kk = 0; kk < kpt_blocks; ++kk) {
-                bool any_hi = false;
-                for (int j = kk * 64; j < (kk + 1) * 64 && j < cw.k_per_tap; ++j) any_hi |= has_hi[size_t(t) * cw.k_per_tap + j] != 0;
-                if (any_hi) m &= ~(1ull << kk);
-            }
-        cw.lo_mask = kpt_blocks == 64 ? m : (m & ((1ull << kpt_blocks) - 1));
-    }
-    VF_TRY(ralloc(h, &cw.w, B.size()));
-    VF_TRY(ralloc(h, &cw.scale, size_t(n_out)));
-    VF_TRY(ralloc(h, &cw.bias, size_t(n_out)));
-    VF_CUDA(cudaMemcpy(cw.w, B.data(), B.size() * sizeof(__half), cudaMemcpyHostToDevice));
-    VF_CUDA(cudaMemcpy(cw.scale, sc.data(), n_out * sizeof(float), cudaMemcpyHostToDevice));
-    VF_CUDA(cudaMemcpy(cw.bias, bi.data(), n_out * sizeof(float), cudaMemcpyHostToDevice));
-    return VF_OK;
-}
-
-struct BnFold { std::vector<float> scale, shift; };
-static bool bn_fold(const TensorTable& T, const std::string& p, int c, BnFold* f) {
-    const float *g = T.get(p + ".weight", c), *b = T.get(p + ".bias", c), *m = T.get(p + ".running_mean", c),
-                *v = T.get(p + ".running_var", c);
-    if (!g || !b || !m || !v) return false;
-    f->scale.resize(c); f->shift.resize(c);
-    for (int i = 0; i < c; ++i) {
-        const float s = g[i] / sqrtf(v[i] + 1e-5f);
-        f->scale[i] = s;
-        f->shift[i] = b[i] - m[i] * s;
-    }
-    return true;
-}
-
-// stride-1 kh x kw conv whose input rows have `pitch` channels with the conv's channel c stored at column chan(c):
-// taps = kernel rows, each a run of kw*pitch elements starting (kw/2) positions to the left.
-static int prep_same_conv(vf_raft* h, ConvW& cw, const TensorTable& T, const std::string& name, int co, int ci, int kh,
-                          int kw, int pitch, const std::function<int(int)>& chan, int n_out, const BnFold* bn,
-                          float extra_scale = 1.f, const std::function<int(int)>& chan_lo = nullptr, int nsplit = -1) {
-    const float* w = T.get(name + ".weight", int64_t(co) * ci * kh * kw);
-    const float* b = T.get(name + ".bias", co);
-    if (!w || !b) return fail(VF_ERR_INVALID, "raft_create: missing or mis-shaped tensor '%s'", name.c_str());
-    cw.ntaps = kh; cw.k_per_tap = kw * pitch;
-    cw.dh.clear(); cw.dw0.clear();
-    for (int a = 0; a < kh; ++a) { cw.dh.push_back(a - kh / 2); cw.dw0.push_back(-(kw / 2)); }
-    const int kpt = cw.k_per_tap;
-    return upload_conv(h, cw, w, b, co, ci, kh, kw, n_out, kh * kpt,
-                       [=](int a, int d, int c) { return a * kpt + d * pitch + chan(c); },
-                       bn ? bn->scale.data() : nullptr, bn ? bn->shift.data() : nullptr, extra_scale,
-                       chan_lo ? std::function<int(int, int, int)>([=](int a, int d, int c) {
-                           const int k = chan_lo(c);
-                           return k < 0 ? -1 : a * kpt + d * pitch + k;
-                       }) : nullptr, nsplit);
-}
-// same, but every (kh, kw) position is its own tap reading `ci` channels at column offset 0 of rows with a wider pitch
-// (dup: the operand row holds [x_hi (ci) | x_lo (ci)], the weight is written to both halves)
-static int prep_unmerged_conv(vf_raft* h, ConvW& cw, const TensorTable& T, const std::string& name, int co, int ci, int kh,
-                              int kw, int n_out, bool dup, float extra_scale = 1.f, int nsplit = -1) {
-    const float* w = T.get(name + ".weight", int64_t(co) * ci * kh * kw);
-    const float* b = T.get(name + ".bias", co);
-    if (!w || !b) return fail(VF_ERR_INVALID, "raft_create: missing or mis-shaped tensor '%s'", name.c_str());
-    const int kpt = dup ? 2 * ci : ci;
-    cw.ntaps = kh * kw; cw.k_per_tap = kpt;
-    cw.dh.clear(); cw.dw0.clear();
-    for (int a = 0; a < kh; ++a)
-        for (int d = 0; d < kw; ++d) { cw.dh.push_back(a - kh / 2); cw.dw0.push_back(d - kw / 2); }
-    return upload_conv(h, cw, w, b, co, ci, kh, kw, n_out, kh * kw * kpt,
-                       [=](int a, int d, int c) { return (a * kw + d) * kpt + c; }, nullptr, nullptr, extra_scale,
-                       dup ? std::function<int(int, int, int)>([=](int a, int d, int c) { return (a * kw + d) * kpt + ci + c; })
-                           : nullptr, nsplit);
-}
-// stride-2 k x k conv (pad k/2) on the phase repack of its input: phase volume row q holds x[2(q-B)+p] with B =
-// border-before (2 for k=7, 1 for k=3); filter index = 2a + p - 1 for tap a (k=7: a in 0..3, k=3: a in 0..1).
-// Row layout: `pitch` channels per position, channel c of phase (ph,pw) at (ph*2+pw)*phase_stride + c, and -- when the
-// activation is a split-fp16 pair -- its lo half `lo_off` columns further (lo_off < 0: single fp16).
-static int prep_stride2_conv(vf_raft* h, ConvW& cw, const TensorTable& T, const std::string& name, int co, int ci, int k,
-                             int pitch, int phase_stride, int lo_off, int n_out, const BnFold* bn) {
-    const float* w = T.get(name + ".weight", int64_t(co) * ci * k * k);
-    const float* b = T.get(name + ".bias", co);
-    if (!w || !b) return fail(VF_ERR_INVALID, "raft_create: missing or mis-shaped tensor '%s'", name.c_str());
-    const int na = (k == 7) ? 4 : 2, before = (k == 7) ? 2 : 1;
-    cw.ntaps = na; cw.k_per_tap = na * pitch;
-    cw.dh.clear(); cw.dw0.clear();
-    for (int a = 0; a < na; ++a) { cw.dh.push_back(a - before); cw.dw0.push_back(-before); }
-    const int kpt = cw.k_per_tap;
-    // invert (kh, kw) -> (a, ph), (bq, pw): kh = 2a + ph - 1
-    auto col = [=](int kh, int kw, int c) {
-        const int a = (kh + 1) / 2, ph = (kh + 1) % 2, bq = (kw + 1) / 2, pw = (kw + 1) % 2;
-        return a * kpt + bq * pitch + (ph * 2 + pw) * phase_stride + c;
-    };
-    return upload_conv(h, cw, w, b, co, ci, k, k, n_out, na * kpt, col,
-                       bn ? bn->scale.data() : nullptr, bn ? bn->shift.data() : nullptr, 1.f,
-                       lo_off >= 0 ? std::function<int(int, int, int)>([=](int kh, int kw, int c) { return col(kh, kw, c) + lo_off; })
-                                   : nullptr);
-}
-// 1x1 stride-2 downsample: phase (0,0) of the repacked row = its first 2*ci channels [hi ci | lo ci]
-static int prep_down_conv(vf_raft* h, ConvW& cw, const TensorTable& T, const std::string& name, int co, int ci, int n_out,
-                          const BnFold* bn) {
-    const float* w = T.get(name + ".weight", int64_t(co) * ci);
-    const float* b = T.get(name + ".bias", co);
-    if (!w || !b) return fail(VF_ERR_INVALID, "raft_create: missing or mis-shaped tensor '%s'", name.c_str());
-    cw.ntaps = 1; cw.k_per_tap = 2 * ci;
-    cw.dh = {0}; cw.dw0 = {0};
-    return upload_conv(h, cw, w, b, co, ci, 1, 1, n_out, cw.k_per_tap, [=](int, int, int c) { return c; },
-                       bn ? bn->scale.data() : nullptr, bn ? bn->shift.data() : nullptr, 1.f,
-                       [=](int, int, int c) { return ci + c; });
-}
-
 // Both encoders keep their activations as split-fp16 pairs, rows = [hi C | lo C]: the instance-norm encoder's are
 // written by the normalisation kernels (fp32 conv outputs), the batch-norm encoder's by the GEMM epilogue's split
 // output (norms folded into scale / bias).  The stem reads the split input phase volume.
@@ -267,11 +99,11 @@ static int prep_encoder(vf_raft* h, vf_raft::Enc& e, const TensorTable& T, const
         bn = &f; return VF_OK;
     };
     auto same3 = [&](ConvW& cw, const std::string& name, int co, int ci) -> int {
-        return prep_same_conv(h, cw, T, name, co, ci, 3, 3, 2 * ci, ident, co, bn, 1.f, [=](int c) { return ci + c; });
+        return prep_same_conv(h->ca, cw, T, name, co, ci, 3, 3, 2 * ci, ident, co, bn, 1.f, [=](int c) { return ci + c; });
     };
     VF_TRY(fold(p + ".norm1", 64));
     // stem: input phase rows = [16 hi | 16 lo], 4 (3 used) channels per phase
-    VF_TRY(prep_stride2_conv(h, e.conv1, T, p + ".conv1", 64, 3, 7, 32, 4, 16, 64, bn));
+    VF_TRY(prep_stride2_conv(h->ca, e.conv1, T, p + ".conv1", 64, 3, 7, 32, 4, 16, 64, bn));
     for (int blk = 0; blk < 2; ++blk)
         for (int cv = 0; cv < 2; ++cv) {
             const std::string b = p + ".layer1." + std::to_string(blk);
@@ -286,9 +118,9 @@ static int prep_encoder(vf_raft* h, vf_raft::Enc& e, const TensorTable& T, const
         ConvW& dn = L == 0 ? e.l2down : e.l3down;
         ConvW* rest = L == 0 ? e.l2 : e.l3;
         VF_TRY(fold(lp + ".0.norm1", co));
-        VF_TRY(prep_stride2_conv(h, c1, T, lp + ".0.conv1", co, ci, 3, 8 * ci, 2 * ci, ci, co, bn));
+        VF_TRY(prep_stride2_conv(h->ca, c1, T, lp + ".0.conv1", co, ci, 3, 8 * ci, 2 * ci, ci, co, bn));
         VF_TRY(fold(lp + ".0.downsample.1", co));
-        VF_TRY(prep_down_conv(h, dn, T, lp + ".0.downsample.0", co, ci, co, bn));
+        VF_TRY(prep_down_conv(h->ca, dn, T, lp + ".0.downsample.0", co, ci, co, bn, ci));
         VF_TRY(fold(lp + ".0.norm2", co));
         VF_TRY(same3(rest[0], lp + ".0.conv2", co, co));
         VF_TRY(fold(lp + ".1.norm1", co));
@@ -296,29 +128,16 @@ static int prep_encoder(vf_raft* h, vf_raft::Enc& e, const TensorTable& T, const
         VF_TRY(fold(lp + ".1.norm2", co));
         VF_TRY(same3(rest[2], lp + ".1.conv2", co, co));
     }
-    VF_TRY(prep_same_conv(h, e.conv2, T, p + ".conv2", out_dim, 128, 1, 1, 256, ident, out_dim, nullptr, 1.f,
+    VF_TRY(prep_same_conv(h->ca, e.conv2, T, p + ".conv2", out_dim, 128, 1, 1, 256, ident, out_dim, nullptr, 1.f,
                           [](int c) { return 128 + c; }));
     return VF_OK;
 }
 
-// out_mode: 0 fp16, 1 fp32, 2 split-fp16 pair (hi at column n, lo at column split_off + n of the same rows)
-// lead: guard rows in front of X and out (both pointers are past them); the GEMM covers them and writes them as zeros
+// the shared conv launch (conv2d.h), counted in the handle's launch total
 static int run_conv(vf_raft* h, const ConvW& cw, const __half* X, int pitch, const Vol2& v, void* out, int ldo, int out_mode,
                     int act, cudaStream_t s, int split_off = 0, int lead = 0) {
-    ConvGeom g;
-    memset(&g, 0, sizeof(g));
-    g.ntaps = cw.ntaps; g.k_per_tap = cw.k_per_tap; g.nsplit = cw.nsplit; g.lo_mask = cw.lo_mask;
-    for (int j = 0; j < cw.ntaps; ++j) g.tap_off[j] = cw.dh[j] * v.Wp + cw.dw0[j];
-    g.mask = 1; g.row0 = lead;
-    g.Tp = 1; g.Hp = v.Hp; g.Wp = v.Wp; g.t0 = 0; g.t1 = 1; g.h0 = v.h0; g.h1 = v.h1; g.w0 = v.w0; g.w1 = v.w1;
-    X -= size_t(lead) * pitch;
-    out = static_cast<char*>(out) - size_t(lead) * ldo * (out_mode == 1 ? 4 : 2);
-    GemmEpi ep;
-    memset(&ep, 0, sizeof(ep));
-    ep.out = out; ep.ldo = ldo; ep.out_f32 = out_mode == 1; ep.bias = cw.bias; ep.scale = cw.scale; ep.act = act;
-    ep.split_off = out_mode == 2 ? split_off : 0;
     h->launches += 1;
-    return conv_gemm_f16(X, pitch, v.rows() + lead, cw.w, cw.n_out, g, ep, s);
+    return run_conv(cw, X, pitch, v, out, ldo, out_mode, act, s, split_off, lead);
 }
 
 // BasicEncoder.forward on m frames whose (split) stem phase volume is in h->s0; the 256-channel output is written in
@@ -360,7 +179,7 @@ static int run_encoder(vf_raft* h, const vf_raft::Enc& e, bool inst, int m, int 
     // a stride-2 residual block: vin (Cin) -> vout (Cout)
     auto down_block = [&](const ConvW& c1, const ConvW& dn, const ConvW& c2, const Vol2& vin, const Vol2& vout, int Cin,
                           int Cout) -> int {
-        VF_TRY(raft_phase_repack(x, vin, 2 * Cin, ph, vout, s));
+        VF_TRY(conv2d_phase_repack(x, vin, 2 * Cin, ph, vout, s));
         h->launches += 1;
         if (inst) {
             VF_TRY(run_conv(h, c1, ph, 8 * Cin, vout, rf, Cout, 1, VF_ACT_NONE, s));
@@ -409,22 +228,23 @@ int vf_raft_create(vf_raft_t** out, const vf_named_tensor* tensors, int n_tensor
     auto ident = [](int c) { return c; };
     {
         const char* e = getenv("VF_RAFT_FAST");
-        h->wsplit = (e && e[0] == '1') ? 1 : 2;
+        h->ca.wsplit = (e && e[0] == '1') ? 1 : 2;
     }
+    h->ca.alloc = [h](void** p, size_t count, size_t elem) { return ralloc(h, reinterpret_cast<char**>(p), count * elem); };
     auto body = [&]() -> int {
         VF_TRY(prep_encoder(h, h->enc[0], T, "fnet", false, 256));
         VF_TRY(prep_encoder(h, h->enc[1], T, "cnet", true, 256));
         const std::string u = "update_block.";
-        VF_TRY(prep_same_conv(h, h->convc1, T, u + "encoder.convc1", 256, 324, 1, 1, CF, ident, 256, nullptr, 1.f,
+        VF_TRY(prep_same_conv(h->ca, h->convc1, T, u + "encoder.convc1", 256, 324, 1, 1, CF, ident, 256, nullptr, 1.f,
                               [](int c) { return RAFT_CF_LO + c; }));                // lo half of the correlation features
         auto lo256 = [](int c) { return 256 + c; };
-        VF_TRY(prep_same_conv(h, h->convc2, T, u + "encoder.convc2", 192, 256, 3, 3, 512, ident, 192, nullptr, 1.f, lo256));
-        VF_TRY(prep_same_conv(h, h->convf1, T, u + "encoder.convf1", 128, 2, 7, 7, 8, ident, 128, nullptr, 1.f,
+        VF_TRY(prep_same_conv(h->ca, h->convc2, T, u + "encoder.convc2", 192, 256, 3, 3, 512, ident, 192, nullptr, 1.f, lo256));
+        VF_TRY(prep_same_conv(h->ca, h->convf1, T, u + "encoder.convf1", 128, 2, 7, 7, 8, ident, 128, nullptr, 1.f,
                               [](int c) { return 2 + c; }));                         // flow8 = (fx_hi, fy_hi, fx_lo, fy_lo, ...)
-        VF_TRY(prep_same_conv(h, h->convf2, T, u + "encoder.convf2", 64, 128, 3, 3, 256, ident, 64, nullptr, 1.f,
+        VF_TRY(prep_same_conv(h->ca, h->convf2, T, u + "encoder.convf2", 64, 128, 3, 3, 256, ident, 64, nullptr, 1.f,
                               [](int c) { return 128 + c; }));
         // reads c2f rows = [cor 192 | flo 64 | cor_lo 192 | flo_lo 64]
-        VF_TRY(prep_same_conv(h, h->convm, T, u + "encoder.conv", 126, 256, 3, 3, 512, ident, 128, nullptr, 1.f, lo256));
+        VF_TRY(prep_same_conv(h->ca, h->convm, T, u + "encoder.conv", 126, 256, 3, 3, 512, ident, 128, nullptr, 1.f, lo256));
         // (columns 126, 127 of the motion block hold the flow: raft_flow_fill rewrites them after this conv's 128-wide
         // store.  Clipping the store at 126 columns does not work: a TMA store view whose row is not a multiple of 16 bytes
         // damaged the two neighbouring elements -- measured 5e-3 flow error.)
@@ -450,14 +270,14 @@ int vf_raft_create(vf_raft_t** out, const vf_named_tensor* tensors, int n_tensor
             memcpy(bzr.data() + 128, br, sizeof(float) * 128);
             const vf_named_tensor tmp[2] = {{"zr.weight", wzr.data(), int64_t(wzr.size())}, {"zr.bias", bzr.data(), 256}};
             const TensorTable TT{tmp, 2};
-            VF_TRY(prep_same_conv(h, zr, TT, "zr", 256, 384, kh, kw, HX, gmap, 256, nullptr, 1.f, gmap_lo));
-            VF_TRY(prep_same_conv(h, qq, T, u + "gru.convq" + sfx, 128, 384, kh, kw, HX, gmap, 128, nullptr, 1.f, gmap_lo));
+            VF_TRY(prep_same_conv(h->ca, zr, TT, "zr", 256, 384, kh, kw, HX, gmap, 256, nullptr, 1.f, gmap_lo));
+            VF_TRY(prep_same_conv(h->ca, qq, T, u + "gru.convq" + sfx, 128, 384, kh, kw, HX, gmap, 128, nullptr, 1.f, gmap_lo));
         }
-        VF_TRY(prep_unmerged_conv(h, h->fh1, T, u + "flow_head.conv1", 256, 128, 3, 3, 256, true));    // reads [h_hi | h_lo]
-        VF_TRY(prep_same_conv(h, h->fh2, T, u + "flow_head.conv2", 2, 256, 3, 3, 512, ident, 8, nullptr, 1.f, lo256));
+        VF_TRY(prep_unmerged_conv(h->ca, h->fh1, T, u + "flow_head.conv1", 256, 128, 3, 3, 256, true));    // reads [h_hi | h_lo]
+        VF_TRY(prep_same_conv(h->ca, h->fh2, T, u + "flow_head.conv2", 2, 256, 3, 3, 512, ident, 8, nullptr, 1.f, lo256));
         // the convex-upsampling mask is three orders of magnitude less sensitive (4e-6 from fp16 weights): single fp16
-        VF_TRY(prep_unmerged_conv(h, h->mk0, T, u + "mask.0", 256, 128, 3, 3, 256, true, 1.f, 1));
-        VF_TRY(prep_same_conv(h, h->mk2, T, u + "mask.2", 576, 256, 1, 1, 256, ident, 576, nullptr, 0.25f, nullptr, 1));   // .25 * mask
+        VF_TRY(prep_unmerged_conv(h->ca, h->mk0, T, u + "mask.0", 256, 128, 3, 3, 256, true, 1.f, 1));
+        VF_TRY(prep_same_conv(h->ca, h->mk2, T, u + "mask.2", 576, 256, 1, 1, 256, ident, 576, nullptr, 0.25f, nullptr, 1));   // .25 * mask
         {
             const size_t np8 = (size_t(h->max_h / 8) * (h->max_w / 8) + 7) / 8 * 8 + 64;
             std::vector<float> s16(np8, 1.0f / 16.0f);     // corr / sqrt(256) (corr.py:60)

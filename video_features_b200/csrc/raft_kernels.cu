@@ -51,24 +51,6 @@ __global__ void raft_input_pack_kernel(const TIn* __restrict__ img, int n, int H
     for (int i = 0; i < 4; ++i) o[i] = reinterpret_cast<const uint4*>(vals)[i];
 }
 
-// space-to-depth for a stride-2 3x3 (pad 1) consumer: out[q][(ph*2+pw)*C + c] = in_valid[2(q-1)+ph][2(q'-1)+pw][c]
-// (zero outside the valid region); out is a border-1 volume at half resolution with 4*C channels.
-__global__ void phase_repack_kernel(const __half* __restrict__ in, Vol2 vi, int C, __half* __restrict__ out, Vol2 vo) {
-    const int cg = C >> 3;
-    const int64_t idx = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-    const int64_t total = int64_t(vo.n) * vo.Hp * vo.Wp * 4 * cg;
-    if (idx >= total) return;
-    const int c8 = int(idx % cg);
-    const int p = int((idx / cg) % 4);
-    const int64_t pos = idx / (4 * cg);
-    const int wq = int(pos % vo.Wp), hq = int((pos / vo.Wp) % vo.Hp), b = int(pos / (int64_t(vo.Wp) * vo.Hp));
-    const int y = 2 * (hq - 1) + (p >> 1), x = 2 * (wq - 1) + (p & 1);     // valid-region coordinates of the input
-    uint4 v = make_uint4(0, 0, 0, 0);
-    if (y >= 0 && y < vi.h1 - vi.h0 && x >= 0 && x < vi.w1 - vi.w0)
-        v = __ldg(reinterpret_cast<const uint4*>(in + ((int64_t(b) * vi.Hp + y + vi.h0) * vi.Wp + x + vi.w0) * C + c8 * 8));
-    *reinterpret_cast<uint4*>(out + pos * (4 * C) + p * C + c8 * 8) = v;
-}
-
 // InstanceNorm2d statistics: per (sample, channel) sum and sum of squares over the valid region.  grid (H, n): one block
 // per image row, block = C * S threads (S position phases per channel); fp32 partials per thread over <= W/S values, the
 // S partials and the rows are combined in double.
@@ -495,11 +477,6 @@ int raft_input_pack(const void* img, int is_u8, int chw, int n, int Hs, int Ws, 
     const int64_t total = int64_t(n) * Hq * Wq;      // rows of 32 channels (16 hi | 16 lo)
     if (is_u8) raft_input_pack_kernel<uint8_t><<<nb(total, 256), 256, 0, s>>>(static_cast<const uint8_t*>(img), n, Hs, Ws, pad_top, pad_left, H, W, chw, out, Hq, Wq);
     else       raft_input_pack_kernel<float><<<nb(total, 256), 256, 0, s>>>(static_cast<const float*>(img), n, Hs, Ws, pad_top, pad_left, H, W, chw, out, Hq, Wq);
-    LAUNCH_CHECK();
-}
-int raft_phase_repack(const __half* in, const Vol2& vi, int C, __half* out, const Vol2& vo, cudaStream_t s) {
-    const int64_t total = int64_t(vo.n) * vo.Hp * vo.Wp * 4 * (C / 8);
-    phase_repack_kernel<<<nb(total, 256), 256, 0, s>>>(in, vi, C, out, vo);
     LAUNCH_CHECK();
 }
 int raft_instnorm_stats(const float* x, const Vol2& v, int C, double* stats, cudaStream_t s) {

@@ -4,6 +4,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "conv2d.h"   // Vol2
+
 namespace vf {
 
 // Row layout of the GRU operand buffers hx / qx (768 columns = 12 K blocks of 64, each purely hi or purely lo):
@@ -15,17 +17,8 @@ constexpr int RAFT_HX = 768, RAFT_HX_MOTION = 512, RAFT_HX_FLOW = 638, RAFT_HX_L
 // correlation features (324 = 4 levels x 81): [hi 324 + 60 zero | lo 324 + 60 zero]
 constexpr int RAFT_CF = 768, RAFT_CF_LO = 384;
 
-// zero-bordered 2-D volume [n][Hp][Wp][C]; valid region [h0,h1) x [w0,w1)
-struct Vol2 {
-    int n, Hp, Wp, h0, h1, w0, w1;
-    int64_t rows() const { return int64_t(n) * Hp * Wp; }
-    int H() const { return h1 - h0; }
-    int W() const { return w1 - w0; }
-};
-
 int raft_input_pack(const void* img, int is_u8, int chw, int n, int Hs, int Ws, int pad_top, int pad_left, int H, int W,
                     __half* out, int Hq, int Wq, cudaStream_t s);
-int raft_phase_repack(const __half* in, const Vol2& vi, int C, __half* out, const Vol2& vo, cudaStream_t s);
 int raft_instnorm_stats(const float* x, const Vol2& v, int C, double* stats, cudaStream_t s);
 int raft_instnorm_apply(const float* a, const double* a_stats, const __half* res_h, const float* res_raw,
                         const double* res_stats, __half* out, const Vol2& v, int C, cudaStream_t s);

@@ -116,6 +116,23 @@ def _(handle, x):
     return x.new_empty((x.shape[0], 1024), dtype=torch.float32)
 
 
+@torch.library.custom_op("vfeat::resnet_forward", mutates_args=())
+def resnet_forward(handle: int, dim: int, x: torch.Tensor) -> torch.Tensor:
+    """`model(x)` of torchvision resnet{depth} with fc = Identity (vf_resnet_forward_f32): (n,3,224,224) fp32 normalised
+    on the device -> (n, dim) fp32."""
+    _need_cuda(x)
+    assert x.dtype == torch.float32 and x.dim() == 4 and tuple(x.shape[1:]) == (3, 224, 224)
+    out = torch.empty((x.shape[0], dim), device=x.device, dtype=torch.float32)
+    with torch.cuda.device(x.device):
+        check(lib().vf_resnet_forward_f32(C.c_void_p(handle), x.data_ptr(), x.shape[0], out.data_ptr(), _stream()))
+    return out
+
+
+@resnet_forward.register_fake
+def _(handle, dim, x):
+    return x.new_empty((x.shape[0], dim), dtype=torch.float32)
+
+
 # ----------------------------------------------------------------------------- transforms
 @torch.library.custom_op("vfeat::resize_u8", mutates_args=())
 def resize_u8(frames: torch.Tensor, out_h: int, out_w: int, filter: int) -> torch.Tensor:

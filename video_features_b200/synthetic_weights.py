@@ -82,6 +82,68 @@ def clip_vit_b32_state_dict(seed: int = 0, outliers: bool = False, patch: int = 
     return sd
 
 
+# torchvision resnet{depth}: block type and blocks per stage (torchvision/models/resnet.py)
+RESNET_BLOCKS = {18: ("basic", (2, 2, 2, 2)), 34: ("basic", (3, 4, 6, 3)), 50: ("bottleneck", (3, 4, 6, 3)),
+                 101: ("bottleneck", (3, 4, 23, 3)), 152: ("bottleneck", (3, 8, 36, 3))}
+
+
+def resnet_feature_dim(depth: int) -> int:
+    return 512 if RESNET_BLOCKS[depth][0] == "basic" else 2048
+
+
+def resnet_conv_shapes(depth: int) -> "OrderedDict[str, tuple]":
+    """torchvision key prefix of every conv -> (cout, cin, k), with the BN that follows it at the same prefix with
+    ``conv`` -> ``bn`` (``downsample.0`` -> ``downsample.1``)."""
+    kind, blocks = RESNET_BLOCKS[depth]
+    exp = 1 if kind == "basic" else 4
+    shapes: "OrderedDict[str, tuple]" = OrderedDict()
+    shapes["conv1"] = (64, 3, 7)
+    cin = 64
+    for li, nb in enumerate(blocks):
+        planes = 64 << li
+        for b in range(nb):
+            p = f"layer{li + 1}.{b}"
+            if kind == "basic":
+                shapes[p + ".conv1"] = (planes, cin, 3)
+                shapes[p + ".conv2"] = (planes, planes, 3)
+            else:
+                shapes[p + ".conv1"] = (planes, cin, 1)
+                shapes[p + ".conv2"] = (planes, planes, 3)
+                shapes[p + ".conv3"] = (planes * 4, planes, 1)
+            if b == 0 and (li > 0 or cin != planes * exp):
+                shapes[p + ".downsample.0"] = (planes * exp, cin, 1)
+            cin = planes * exp
+    return shapes
+
+
+def resnet_bn_name(conv: str) -> str:
+    return conv[:-1] + "1" if conv.endswith("downsample.0") else conv.replace("conv", "bn")
+
+
+def resnet_state_dict(depth: int, seed: int = 0) -> "OrderedDict[str, torch.Tensor]":
+    """torchvision ``resnet{depth}`` key layout, fp32 (``fc.*`` and ``num_batches_tracked`` included, as in a real
+    checkpoint).  He-scaled convs and mild BN statistics; the last BN gain of every residual branch is damped to
+    0.2 (bn2 of a BasicBlock, bn3 of a Bottleneck), so that the residual stream stays O(1) through 50 blocks instead of
+    growing with depth (tests/test_resnet_cpu.py holds the per-stage RMS in a band)."""
+    g = torch.Generator().manual_seed(seed)
+    kind = RESNET_BLOCKS[depth][0]
+    last = ".bn2" if kind == "basic" else ".bn3"
+    sd: "OrderedDict[str, torch.Tensor]" = OrderedDict()
+    for name, (co, ci, k) in resnet_conv_shapes(depth).items():
+        sd[name + ".weight"] = torch.randn(co, ci, k, k, generator=g) * (2.0 / (ci * k * k)) ** 0.5
+        bn = resnet_bn_name(name)
+        gain = 0.2 if bn.endswith(last) else 1.0
+        sd[bn + ".weight"] = gain * (1.0 + 0.1 * torch.randn(co, generator=g))
+        sd[bn + ".bias"] = 0.05 * torch.randn(co, generator=g)
+        sd[bn + ".running_mean"] = 0.05 * torch.randn(co, generator=g)
+        sd[bn + ".running_var"] = 1.0 + 0.1 * torch.rand(co, generator=g)
+        sd[bn + ".num_batches_tracked"] = torch.tensor(0, dtype=torch.int64)
+    d = resnet_feature_dim(depth)
+    sd["fc.weight"] = torch.randn(1000, d, generator=g) * d ** -0.5
+    sd["fc.bias"] = torch.zeros(1000)
+    return sd
+
+
 def parse_env(value: str):
     """``VF_CLIP_SYNTHETIC`` value -> (seed, outliers): "3", "3:outliers", "" (seed 0)."""
     head, _, tail = (value or "").partition(":")
